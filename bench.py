@@ -8,6 +8,7 @@ is reported in the extra key ``allreduce_busbw_gbs``.
     python bench.py --gpus N --steps K --warmup W            # N=1 directly
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...   # N>1
     python bench.py --impl reference                          # reference arm
+    python bench.py ... --dump-outputs DIR                    # + the state after the last timed step, DIR/*.npy
 
 * device-timed with CUDA events on the launching stream, barrier + synchronize on both
   sides, max over ranks; W untimed warm-up steps, exactly K timed steps;
@@ -63,7 +64,11 @@ def main() -> int:
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--grid", type=int, default=GRID)
     ap.add_argument("--no-sweep", action="store_true", help="skip the allreduce sweep extras")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the model state after the last timed step to DIR/<field>.npy (see dump_outputs)")
     ns = ap.parse_args()
+    if ns.steps < 1:
+        ap.error("--steps must be at least 1")
     if ns.impl == "reference":
         return reference_arm()
 
@@ -162,6 +167,8 @@ def main() -> int:
         gpu_launches = run_steps(K)
         end.record()
         torch.cuda.synchronize()
+        # the state the timed steps left, before the untimed steps below advance it
+        timed_state = [t.clone() for t in model.state] if ns.dump_outputs else None
         if start.elapsed_time(end) < 400:           # keep the GPU under load long enough to sample
             t_end = time.time() + 0.5
             while time.time() < t_end:
@@ -300,8 +307,37 @@ def main() -> int:
         if sweep is not None:
             out["allreduce_busbw_gbs"] = sweep
         print(json.dumps(out))
+    if ns.dump_outputs:
+        dump_outputs(ns.dump_outputs, model, timed_state)
     m.flush()
     return 0
+
+
+DUMP_SAMPLE = 1 << 21          # values per field: 6 float32 fields of 8 MiB, 48 MiB in all
+DUMP_SEED = 0
+
+
+def dump_outputs(directory, model, state):
+    """Write ``state`` (h, u, v, dh, du, dv: what ``model.multistep`` leaves a caller) as
+    ``directory/<field>.npy`` in float32, so that two builds can be compared output for output.
+    Each field is the global (ny + 2, nx + 2) array including its halo ring, gathered on rank 0.
+    A field of more than DUMP_SAMPLE values is written as the values at DUMP_SAMPLE sorted flat
+    indices drawn without replacement by numpy's default_rng(DUMP_SEED): the same indices for
+    every run on the same grid, whatever the number of GPUs."""
+    import numpy as np
+
+    index = None
+    for name, local in zip(model.state._fields, state):
+        field = model.gather_global(local)          # collective: every rank takes part
+        if field is None:
+            continue
+        arr = field.float().cpu().numpy()
+        if arr.size > DUMP_SAMPLE:
+            if index is None:
+                index = np.sort(np.random.default_rng(DUMP_SEED).choice(arr.size, DUMP_SAMPLE, replace=False))
+            arr = arr.reshape(-1)[index]
+        os.makedirs(directory, exist_ok=True)
+        np.save(os.path.join(directory, f"{name}.npy"), arr)
 
 
 def correctness_checks(m, MPI, comm, dev):

@@ -1,7 +1,5 @@
 """Port of /root/reference/tests/collective_ops/test_barrier.py."""
 
-import os
-import tempfile
 import time
 
 import torch
@@ -12,11 +10,22 @@ from mpi4jax_b200 import MPI
 comm = MPI.COMM_WORLD
 
 
-def test_barrier(device):
+def _path_of_rank0(path):
+    """rank 0's file name -> all ranks (uint8 bcast through the public op)."""
+    buf = torch.zeros(4096, dtype=torch.uint8)
+    if comm.Get_rank() == 0:
+        raw = str(path).encode()
+        buf[: len(raw)] = torch.tensor(list(raw), dtype=torch.uint8)
+    buf = m.bcast(buf.to(comm.device), 0, comm=comm).cpu()
+    return bytes(buf[buf != 0].tolist()).decode()
+
+
+def test_barrier(device, tmp_path):
     """Ranks append lines before/after a barrier to one file; all 'start' lines must precede
     all 'done' lines."""
     rank, size = comm.Get_rank(), comm.Get_size()
-    write_to = os.path.join(tempfile.gettempdir(), f"mpi4jax-b200-barrier-{device.type}.txt")
+    # a file of this run's own (a fixed name in the shared temp directory may belong to another user)
+    write_to = _path_of_rank0(tmp_path / f"barrier-{device.type}.txt")
     if rank == 0:
         with open(write_to, "w"):
             pass

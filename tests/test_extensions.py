@@ -186,13 +186,26 @@ def test_large_rooted_ops_and_scan(device, nbytes):
         assert torch.equal(rb.float(), (torch.arange(n, device=device) % 7).float() * size + size * (size - 1) / 2)
 
 
+@pytest.fixture
+def comm_on_device(device, monkeypatch):
+    """COMM_WORLD, or for the CPU case on a machine with a GPU a clone of it that lives on the CPU
+    (symmetric_empty allocates on its communicator's device)."""
+    if device.type == comm.device.type:
+        yield comm
+        return
+    monkeypatch.setenv("MPI4JAX_B200_DEVICE", "cpu")
+    cpu_comm = comm.Clone()
+    yield cpu_comm
+    cpu_comm.Free()
+
+
 @pytest.mark.parametrize("dtype", [torch.float32, torch.bfloat16, torch.float16])
 @pytest.mark.parametrize("n", [4, 1000, 70_000, (1 << 20) + 8])
-def test_symmetric_tensor_allreduce_in_place(device, dtype, n):
+def test_symmetric_tensor_allreduce_in_place(device, comm_on_device, dtype, n):
     """Extension: tensors allocated in the symmetric heap are reduced in place inside the NVSwitch
     (no staging copy in, none out).  The reference has no registered-memory notion to compare with;
     the oracle is the functional allreduce of the same values."""
-    comm2 = comm
+    comm2 = comm_on_device
     x = m.symmetric_empty((n,), dtype, comm=comm2)
     vals = (torch.arange(n, device=device, dtype=torch.float32) % 13 + rank).to(dtype)
     x.copy_(vals)
