@@ -103,12 +103,10 @@ static inline size_t b2_dtype_size(int dt) {
 //   [flags]      B2_MAX_BLOCKS x B2_MAX_RANKS u32   block-paired barrier flags
 //   [p2p hdr]    P x NSLOT x LANES x 16 B           inbox headers (written by the sender)
 //   [p2p ack]    P x NSLOT x LANES x 4 B            slot credits  (written by the receiver)
-//   [halo flags] 8 sides x 64 B                     fused halo exchange (arrival counters)
 //   [ll]         2 parities x P x ll_cap            flag-in-data allreduce buffers
 //   [p2p slots]  P x NSLOT x slot_bytes             eager/streaming payload ring
 //   [p2p LL]     P x NSLOT x 16 KiB                 small messages, 8-byte {word, seq} stores
-//   [halo bufs]  2 parities x 8 sides x halo_cap
-//   [halo LL]    2 parities x 8 sides x 2*halo_cap  (fused stencil+halo kernels)
+//   [halo LL]    2 parities x 8 sides x halo_ll_cap flag-in-data halo buffers
 //   -- separate, growable segment --
 //   [staging]    2 parities x stage_half            collective staging
 // ---------------------------------------------------------------------------
@@ -116,15 +114,13 @@ struct B2Layout {
   size_t flags_off;
   size_t p2p_hdr_off;
   size_t p2p_ack_off;
-  size_t halo_flag_off;
   size_t ll_off;
   size_t ll_cap;          // bytes per (parity, source) LL buffer (wire bytes = 2x payload)
   size_t p2p_slot_off;
   size_t p2p_slot_bytes;
   size_t p2p_ll_off;      // P x NSLOT x (2 * B2_P2P_LL_MAX): flag-in-data copies of small messages
-  size_t halo_buf_off;
-  size_t halo_cap;        // bytes per (parity, direction)
-  size_t halo_ll_off;     // flag-in-data halo buffers of the fused stencil kernels
+  size_t halo_cap;        // halo payload limit: nfields x max(ny, nx) x 4 B per exchange
+  size_t halo_ll_off;     // flag-in-data halo buffers (b2_halo_ll.cuh)
   size_t halo_ll_cap;     // bytes per (parity, side): 8 B per element
   size_t total;
 };
@@ -142,9 +138,8 @@ struct B2DevComm {
   B2Layout lay;
   // local (non-symmetric) device memory
   unsigned* epoch;                      // [B2_MAX_BLOCKS] per-CTA barrier epochs
-  unsigned* ticket;                     // [0] collective ticket [1] finish ctr [3] halo finish ctr
-                                        // [8..15] halo msgs received per side [16..23] sent per side
-                                        // [5] fused-halo ready ctr [6] finish ctr [32..47] fused rx/tx
+  unsigned* ticket;                     // [0] collective ticket [1] finish ctr [6] halo finish ctr
+                                        // [32..39] halo msgs received per side [40..47] sent per side
   unsigned* p2p_send_seq;               // [P] fragments sent to each destination
   unsigned* p2p_recv_seq;               // [P] fragments consumed from each source
   unsigned* p2p_ctl;                    // [8] arrive counters / any-source election word

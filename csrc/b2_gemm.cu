@@ -335,7 +335,7 @@ extern "C" int b2_gemm_allreduce(B2Comm* c, const void* A, const void* B, void* 
   // more than it gains: 2 GPUs, 4096 x 4096 x 2048: 293 us banded vs 177 us row-major
   // (profiles/r2_gemm_fused_2gpu_banded.log, r1_gemm_allreduce_fused_2gpu.log) -- row-major there
   // until the coordinates are hoisted out of those loops
-  g.raster = c->gemm_raster >= 0 ? c->gemm_raster : (g.fused ? 0 : B2_GEMM_RASTER_GROUP);
+  g.raster = g.fused ? 0 : B2_GEMM_RASTER_GROUP;
   if (g.fused) {
     if (c->dev.stage_mc == nullptr) {
       b2_set_error("gemm_allreduce: multi-rank call needs a multicast-bound staging segment (NVLS)");

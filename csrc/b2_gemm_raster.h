@@ -18,8 +18,8 @@
 #define B2_HD
 #endif
 
-// `group` = G of the description above (0 = row-major); a launch parameter (communicator option
-// "gemm_raster", -1 = pick by shape), B2_GEMM_RASTER_GROUP is the compile-time default.
+// `group` = G of the description above (0 = row-major); a launch parameter (b2_gemm.cu picks it
+// per launch), B2_GEMM_RASTER_GROUP is the compile-time default.
 B2_HD inline void b2_gemm_tile_coords(int tile, int num_m, int num_n, int group, int& m_blk, int& n_blk) {
   if (group > 0) {
     const int G = group;

@@ -9,8 +9,8 @@
 //
 // Here ONE kernel launch exchanges the halos of up to B2_HALO_MAX_FIELDS fields
 // with all EIGHT neighbours in a single phase: strided column pack, NVLink put
-// straight into the neighbour's symmetric receive buffer, one release/acquire
-// flag handshake, halo unpack and the physical wall conditions, all fused.
+// straight into the neighbour's symmetric receive buffer, halo unpack and the
+// physical wall conditions, all fused.
 //
 // Why eight neighbours: the reference's west/north/east/south message order
 // makes every corner halo cell end up with the DIAGONAL neighbour's interior
@@ -20,206 +20,25 @@
 // touches a y wall the wall-row cells of the halo columns come from the W/E
 // neighbours' wall rows, exactly as in the reference's sequence.
 //
-// The work is spread over HALO_CTAS CTAs; every CTA signals every neighbour with
-// one `red.release.sys.add` after its stores, a side is complete when its flag
-// reached (messages received on that side + 1) * HALO_CTAS.  Receive buffers are
-// double-buffered on device-side per-side message counters, so no "ready"
-// handshake is needed and the kernel is CUDA-graph replayable.
+// Every element is pushed as one 8-byte {value, flag} store and the receiver
+// polls the data itself: one NVLink one-way latency (transport: b2_halo_ll.cuh).
+// Receive buffers are double-buffered on device-side per-side message counters,
+// so no "ready" handshake is needed and the kernel is CUDA-graph replayable.
 #include <cstdio>
-#include <cstdlib>
 #include <cstring>
 
 #include "b2_device.cuh"
 #include "b2_halo_ll.cuh"
-#include "b2_launch.cuh"
 #include "b2_runtime.h"
 
 extern "C" void b2_set_error(const char* fmt, ...);
 extern "C" void b2_count_launch(B2Comm* c);
 
 #define HALO_THREADS 256
-#define HALO_CTAS 32
-// receive-buffer / flag index = where the data lands on the RECEIVER
-enum { SIDE_W = 0, SIDE_E, SIDE_S, SIDE_N, SIDE_SW, SIDE_SE, SIDE_NW, SIDE_NE, NSIDES };
-
-__device__ __forceinline__ float* halo_buf(const B2DevComm& c, int rank, unsigned parity, int side) {
-  return (float*)(c.heap[rank] + c.lay.halo_buf_off +
-                  ((size_t)parity * NSIDES + side) * c.lay.halo_cap);
-}
-__device__ __forceinline__ unsigned* halo_flag(const B2DevComm& c, int rank, int side) {
-  return (unsigned*)(c.heap[rank] + c.lay.halo_flag_off) + side * 16;   // 64 B apart
-}
-__device__ __forceinline__ void red_release_add(unsigned* p, unsigned v) {
-  asm volatile("red.release.sys.global.add.u32 [%0], %1;" ::"l"(p), "r"(v) : "memory");
-}
-
-// Per-side message counters (local device memory): c.ticket[8..15] = messages received on
-// each side, c.ticket[16..23] = messages sent towards each direction, c.ticket[3] = finish
-// counter.  A message is complete when the side's flag reached (count + 1) * CTAs; the
-// receive buffer parity is count & 1.  Both ends of a channel count the same messages, so
-// exchanges with different neighbour sets can be mixed freely.
-__global__ void __launch_bounds__(HALO_THREADS) b2_k_halo(const B2DevComm c, const B2HaloDesc d) {
-  b2_pdl_enter();
-  __shared__ unsigned s_rx[NSIDES], s_tx[NSIDES];
-  const int gt = blockIdx.x * blockDim.x + threadIdx.x, gn = gridDim.x * blockDim.x;
-  const int ny = d.ny, nx = d.nx, F = d.nfields;
-  const size_t pitch = (size_t)d.pitch;
-  // rank behind each of my eight sides (source of what I receive there, target of what I send)
-  const int nb[NSIDES] = {d.west, d.east, d.south, d.north, d.sw, d.se, d.nw, d.ne};
-  // my message towards side k lands on the opposite side of the neighbour
-  const int opp[NSIDES] = {SIDE_E, SIDE_W, SIDE_N, SIDE_S, SIDE_NE, SIDE_NW, SIDE_SE, SIDE_SW};
-  if (threadIdx.x < NSIDES) {
-    s_rx[threadIdx.x] = b2_ld_volatile(c.ticket + 8 + threadIdx.x);
-    s_tx[threadIdx.x] = b2_ld_volatile(c.ticket + 16 + threadIdx.x);
-  }
-  __syncthreads();
-#define TXPAR(k) (s_tx[k] & 1u)
-#define RXPAR(k) (s_rx[k] & 1u)
-
-  // ---------------- pack + put ----------------
-  if (d.west >= 0) {   // my column 1 -> west neighbour's east halo (full height)
-    float* dst = halo_buf(c, d.west, TXPAR(SIDE_W), SIDE_E);
-    for (int k = gt; k < F * ny; k += gn) {
-      const int f = k / ny, j = k - f * ny;
-      dst[k] = d.field[f][(size_t)j * pitch + 1];
-    }
-  }
-  if (d.east >= 0) {   // my column nx-2 -> east neighbour's west halo
-    float* dst = halo_buf(c, d.east, TXPAR(SIDE_E), SIDE_W);
-    for (int k = gt; k < F * ny; k += gn) {
-      const int f = k / ny, j = k - f * ny;
-      dst[k] = d.field[f][(size_t)j * pitch + (nx - 2)];
-    }
-  }
-  if (d.south >= 0) {  // my row 1 -> south neighbour's north halo
-    float* dst = halo_buf(c, d.south, TXPAR(SIDE_S), SIDE_N);
-    for (int k = gt; k < F * nx; k += gn) {
-      const int f = k / nx, i = k - f * nx;
-      dst[k] = d.field[f][pitch + i];
-    }
-  }
-  if (d.north >= 0) {  // my row ny-2 -> north neighbour's south halo
-    float* dst = halo_buf(c, d.north, TXPAR(SIDE_N), SIDE_S);
-    for (int k = gt; k < F * nx; k += gn) {
-      const int f = k / nx, i = k - f * nx;
-      dst[k] = d.field[f][(size_t)(ny - 2) * pitch + i];
-    }
-  }
-  if (gt < F) {        // interior corner cells -> diagonal neighbours' corner halo cells
-    const int f = gt;
-    if (d.sw >= 0) halo_buf(c, d.sw, TXPAR(SIDE_SW), SIDE_NE)[f] = d.field[f][pitch + 1];
-    if (d.se >= 0) halo_buf(c, d.se, TXPAR(SIDE_SE), SIDE_NW)[f] = d.field[f][pitch + (nx - 2)];
-    if (d.nw >= 0) halo_buf(c, d.nw, TXPAR(SIDE_NW), SIDE_SE)[f] = d.field[f][(size_t)(ny - 2) * pitch + 1];
-    if (d.ne >= 0)
-      halo_buf(c, d.ne, TXPAR(SIDE_NE), SIDE_SW)[f] = d.field[f][(size_t)(ny - 2) * pitch + (nx - 2)];
-  }
-  __syncthreads();
-  // ---------------- signal, then wait for every side ----------------
-  if (threadIdx.x < NSIDES && nb[threadIdx.x] >= 0) {
-    red_release_add(halo_flag(c, nb[threadIdx.x], opp[threadIdx.x]), 1u);
-    b2_wait_ge(c, halo_flag(c, c.rank, threadIdx.x), (s_rx[threadIdx.x] + 1u) * gridDim.x,
-               B2_OPC_HALO, nb[threadIdx.x]);
-  }
-  __syncthreads();
-
-  // ---------------- unpack (+ wall conditions, examples/shallow_water.py:258-262) ----------------
-  // halo columns: full height where this rank touches a y wall, interior rows otherwise
-  const int jlo = (d.south >= 0) ? 1 : 0, jhi = (d.north >= 0) ? ny - 1 : ny;
-  const bool uwall = !d.periodic_x && d.at_east_wall;
-  if (d.east >= 0) {
-    const float* src = halo_buf(c, c.rank, RXPAR(SIDE_E), SIDE_E);
-    for (int k = gt; k < F * ny; k += gn) {
-      const int f = k / ny, j = k - f * ny;
-      if (j >= jlo && j < jhi) {
-        float val = __ldcv(src + k);
-        if (d.kind[f] == 2 && d.at_north_wall && j == ny - 2) val = 0.f;
-        d.field[f][(size_t)j * pitch + (nx - 1)] = val;
-      }
-    }
-  }
-  if (d.west >= 0) {
-    const float* src = halo_buf(c, c.rank, RXPAR(SIDE_W), SIDE_W);
-    for (int k = gt; k < F * ny; k += gn) {
-      const int f = k / ny, j = k - f * ny;
-      if (j >= jlo && j < jhi) {
-        float val = __ldcv(src + k);
-        if (d.kind[f] == 2 && d.at_north_wall && j == ny - 2) val = 0.f;
-        d.field[f][(size_t)j * pitch] = val;
-      }
-    }
-  }
-  if (d.south >= 0) {   // halo row 0, interior columns (corners come from the diagonals)
-    const float* src = halo_buf(c, c.rank, RXPAR(SIDE_S), SIDE_S);
-    for (int k = gt; k < F * nx; k += gn) {
-      const int f = k / nx, i = k - f * nx;
-      if (i >= 1 && i < nx - 1) {
-        float val = __ldcv(src + k);
-        if (d.kind[f] == 1 && uwall && i == nx - 2) val = 0.f;
-        d.field[f][i] = val;
-      }
-    }
-  }
-  if (d.north >= 0) {
-    const float* src = halo_buf(c, c.rank, RXPAR(SIDE_N), SIDE_N);
-    for (int k = gt; k < F * nx; k += gn) {
-      const int f = k / nx, i = k - f * nx;
-      if (i >= 1 && i < nx - 1) {
-        float val = __ldcv(src + k);
-        if (d.kind[f] == 1 && uwall && i == nx - 2) val = 0.f;
-        d.field[f][(size_t)(ny - 1) * pitch + i] = val;
-      }
-    }
-  }
-  if (gt < F) {
-    const int f = gt;
-    if (d.sw >= 0) d.field[f][0] = __ldcv(halo_buf(c, c.rank, RXPAR(SIDE_SW), SIDE_SW) + f);
-    if (d.se >= 0) d.field[f][nx - 1] = __ldcv(halo_buf(c, c.rank, RXPAR(SIDE_SE), SIDE_SE) + f);
-    if (d.nw >= 0)
-      d.field[f][(size_t)(ny - 1) * pitch] = __ldcv(halo_buf(c, c.rank, RXPAR(SIDE_NW), SIDE_NW) + f);
-    if (d.ne >= 0)
-      d.field[f][(size_t)(ny - 1) * pitch + (nx - 1)] =
-          __ldcv(halo_buf(c, c.rank, RXPAR(SIDE_NE), SIDE_NE) + f);
-  }
-  // cells of the wall row / column that no message writes
-  for (int f = 0; f < F; ++f) {
-    if (d.kind[f] == 1 && uwall)
-      for (int j = gt; j < ny; j += gn)
-        if ((j >= 1 && j < ny - 1) || (j == 0 && d.south < 0) || (j == ny - 1 && d.north < 0))
-          d.field[f][(size_t)j * pitch + (nx - 2)] = 0.f;
-    if (d.kind[f] == 2 && d.at_north_wall)
-      for (int i = gt; i < nx; i += gn)
-        if ((i >= 1 && i < nx - 1) || (i == 0 && d.west < 0) || (i == nx - 1 && d.east < 0))
-          d.field[f][(size_t)(ny - 2) * pitch + i] = 0.f;
-  }
-#undef TXPAR
-#undef RXPAR
-  // last CTA to finish advances the per-side message counters
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    __threadfence();
-    const unsigned old = atomicAdd(c.ticket + 3, 1u);
-    if (old == gridDim.x - 1) {
-      b2_st_volatile(c.ticket + 3, 0u);
-      for (int k = 0; k < NSIDES; ++k)
-        if (nb[k] >= 0) {
-          b2_st_volatile(c.ticket + 8 + k, s_rx[k] + 1u);
-          b2_st_volatile(c.ticket + 16 + k, s_tx[k] + 1u);
-        }
-      __threadfence();
-    }
-  }
-}
-
-// ---------------------------------------------------------------------------------------------
-// Flag-in-data variant (default): same exchange, but every element is pushed as one 8-byte
-// {value, flag} store and the receiver polls the data itself -- no release fence, no arrival
-// counter, one NVLink one-way latency (transport: b2_halo_ll.cuh).
-// ---------------------------------------------------------------------------------------------
-#define HALO_LL_CTAS 16
+#define HALO_MIN_CTAS 16
 
 __global__ void __launch_bounds__(HALO_THREADS) b2_k_halo_ll(const B2DevComm c, const B2HaloDesc d,
                                                              const int fs) {
-  b2_pdl_enter();
   __shared__ unsigned s_rx[FS_NSIDES], s_tx[FS_NSIDES];
   const int gt = blockIdx.x * blockDim.x + threadIdx.x, gn = gridDim.x * blockDim.x;
   const int ny = d.ny, nx = d.nx, F = d.nfields;
@@ -385,20 +204,11 @@ extern "C" int b2_halo_exchange(B2Comm* c, const B2HaloDesc* d, cudaStream_t str
     }
   const int mx = d->ny > d->nx ? d->ny : d->nx;
   const int fs = (mx + 3) / 4 * 4;
-  static int use_ll = -1;
-  if (use_ll < 0) {
-    const char* e = getenv("MPI4JAX_B200_HALO_LL");
-    use_ll = !(e && (e[0] == '0' || e[0] == 'f' || e[0] == 'F'));
-  }
-  if (use_ll && (size_t)d->nfields * fs * sizeof(uint2) <= c->dev.lay.halo_ll_cap) {
-    // about one element per thread and side: the exchange is pure latency, so spread it wide
-    int ctas = (d->nfields * mx + HALO_THREADS - 1) / HALO_THREADS;
-    if (ctas < HALO_LL_CTAS) ctas = HALO_LL_CTAS;
-    if (ctas > 96) ctas = 96;
-    b2_launch(b2_k_halo_ll, ctas, HALO_THREADS, 0, stream, c->dev, *d, fs);
-  }
-  else
-    b2_launch(b2_k_halo, HALO_CTAS, HALO_THREADS, 0, stream, c->dev, *d);
+  // about one element per thread and side: the exchange is pure latency, so spread it wide
+  int ctas = (d->nfields * mx + HALO_THREADS - 1) / HALO_THREADS;
+  if (ctas < HALO_MIN_CTAS) ctas = HALO_MIN_CTAS;
+  if (ctas > 96) ctas = 96;
+  b2_k_halo_ll<<<ctas, HALO_THREADS, 0, stream>>>(c->dev, *d, fs);
   b2_count_launch(c);
   cudaError_t err = cudaGetLastError();
   if (err != cudaSuccess) {

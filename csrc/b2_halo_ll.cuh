@@ -13,9 +13,7 @@
 enum { FS_W = 0, FS_E, FS_S, FS_N, FS_SW, FS_SE, FS_NW, FS_NE, FS_NSIDES };
 
 // ticket words (local device memory)
-#define TK_READY 5     // fused kernels: += 1 per unpacker CTA, reset by the last CTA of the kernel
 #define TK_FIN 6       // finish counter
-#define TK_TILE 7      // fused kernels: dynamic tile scheduler (reset by the last CTA)
 #define TK_RX 32       // [8] messages received per side
 #define TK_TX 40       // [8] messages sent per side
 

@@ -37,17 +37,6 @@ extern "C" void b2_set_logging(int enable) { g_logging = enable ? 1 : 0; }
 extern "C" int b2_get_logging(void) { return g_logging; }
 extern "C" void b2_set_print_callback(b2_print_fn fn) { g_print = fn; }
 extern "C" int b2_launch_count(void) { return g_launches; }
-
-// programmatic dependent launch for the stencil / halo launch chains (csrc/b2_launch.cuh)
-static int g_pdl = -1;
-extern "C" int b2_pdl_enabled(void) {
-  if (g_pdl < 0) {
-    const char* e = getenv("MPI4JAX_B200_PDL");
-    g_pdl = (e && (e[0] == '1' || e[0] == 't' || e[0] == 'T' || ((e[0] == 'o' || e[0] == 'O') && (e[1] == 'n' || e[1] == 'N')))) ? 1 : 0;
-  }
-  return g_pdl;
-}
-extern "C" void b2_set_pdl(int enable) { g_pdl = enable ? 1 : 0; }
 extern "C" void b2_count_launch(B2Comm* c) {
   ++g_launches;
   if (c) ++c->launches;

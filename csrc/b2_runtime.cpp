@@ -358,15 +358,15 @@ static B2Layout make_layout(int nranks, size_t slot_bytes, size_t ll_cap, size_t
   L.flags_off = take((size_t)B2_MAX_BLOCKS * B2_MAX_RANKS * 4);
   L.p2p_hdr_off = take((size_t)nranks * B2_P2P_NSLOT * B2_P2P_MAX_LANES * 16);
   L.p2p_ack_off = take((size_t)nranks * B2_P2P_NSLOT * 4);
-  L.halo_flag_off = take(8 * 64);
   L.ll_cap = round_up(ll_cap, 4096);
   L.ll_off = take(2 * (size_t)nranks * L.ll_cap);
   L.p2p_slot_bytes = round_up(slot_bytes, 4096);
   L.p2p_slot_off = take((size_t)nranks * B2_P2P_NSLOT * L.p2p_slot_bytes);
   L.p2p_ll_off = take((size_t)nranks * B2_P2P_NSLOT * 2 * B2_P2P_LL_MAX);
   L.halo_cap = round_up(halo_cap, 4096);
-  L.halo_buf_off = take(2 * 8 * L.halo_cap);
-  L.halo_ll_cap = 2 * L.halo_cap;
+  // 8 B per element; the extra 4 KiB covers padding each field to a multiple of 4 elements, so every
+  // halo that fits halo_cap as 4-byte floats fits here
+  L.halo_ll_cap = 2 * L.halo_cap + 4096;
   L.halo_ll_off = take(2 * 8 * L.halo_ll_cap);
   L.total = off;
   return L;
@@ -433,7 +433,6 @@ extern "C" B2Comm* b2_comm_create(int device, int rank, int nranks, B2Seg* ctl, 
   c->nvls_min = 64 * 1024 + 1;
   c->bcast_mc_min = 256 * 1024;
   c->nvls_pipeline = 1;
-  c->gemm_raster = -1;
   c->trace = nullptr;
   c->trace_cap = 0;
   // one 512-thread CTA of the collective kernels (<= 128 registers per thread) fits per SM: grids are
@@ -468,7 +467,6 @@ extern "C" int b2_comm_set_tuning(B2Comm* c, long long ll_max, long long oneshot
 extern "C" int b2_comm_set_option(B2Comm* c, const char* key, long long value) {
   if (strcmp(key, "bcast_mc_min") == 0) c->bcast_mc_min = (size_t)value;
   else if (strcmp(key, "nvls_pipeline") == 0) c->nvls_pipeline = value != 0;
-  else if (strcmp(key, "gemm_raster") == 0) c->gemm_raster = (int)value;
   else if (strcmp(key, "trace_ptr") == 0) c->trace = (unsigned long long*)(uintptr_t)value;
   else if (strcmp(key, "trace_cap") == 0) c->trace_cap = (int)value;
   else { b2_set_error("unknown communicator option '%s'", key); return B2_ERR_BAD_ARG; }
@@ -481,7 +479,6 @@ extern "C" long long b2_comm_get_option(B2Comm* c, const char* key) {
   if (strcmp(key, "sm_count") == 0) return c->sm_count;
   if (strcmp(key, "bcast_mc_min") == 0) return (long long)c->bcast_mc_min;
   if (strcmp(key, "nvls_pipeline") == 0) return c->nvls_pipeline ? 1 : 0;
-  if (strcmp(key, "gemm_raster") == 0) return c->gemm_raster < 0 ? 0 : c->gemm_raster;
   b2_set_error("unknown communicator option '%s'", key);
   return -1;
 }

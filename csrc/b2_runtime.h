@@ -54,7 +54,6 @@ struct B2Comm {
   size_t nvls_min;
   size_t bcast_mc_min;          // bcast: root multimem.st from this size on
   int nvls_pipeline;            // software-pipelined NVLS allreduce (default on)
-  int gemm_raster;              // tile order of the persistent GEMM: -1 = compile-time default, 0 = row-major, G = bands
   unsigned long long* trace;    // device buffer for the phase timeline of CTA 0 (scripts/allreduce_phases.py)
   int trace_cap;
   int max_blocks;
@@ -74,8 +73,6 @@ int b2_get_logging(void);
 typedef void (*b2_print_fn)(const char*);
 void b2_set_print_callback(b2_print_fn fn);
 int b2_launch_count(void);
-int b2_pdl_enabled(void);      // programmatic dependent launch of the stencil/halo chain
-void b2_set_pdl(int enable);
 
 // --- device / driver ---------------------------------------------------------
 int b2_init(int device);

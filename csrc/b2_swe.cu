@@ -33,13 +33,11 @@ extern "C" void b2_set_error(const char* fmt, ...);
 extern "C" void b2_count_launch(B2Comm* c);
 
 #include "b2_swe_body.cuh"
-#include "b2_launch.cuh"
 
 __global__ void __launch_bounds__(SWE_THREADS)
 swe_k1_fluxes(B2SweParams p, const float* __restrict__ h, const float* __restrict__ u,
               const float* __restrict__ v, float* __restrict__ fe, float* __restrict__ fn,
               float* __restrict__ q, float* __restrict__ ke) {
-  b2_pdl_enter();
   int j, i0;
   bool m[4];
   if (!swe_map(p, j, i0, m)) return;
@@ -52,7 +50,6 @@ swe_k2_tendencies(B2SweParams p, const float* __restrict__ h, float* __restrict_
                   float* __restrict__ du, float* __restrict__ dv, const float* __restrict__ fe,
                   const float* __restrict__ fn, const float* __restrict__ q,
                   const float* __restrict__ ke) {
-  b2_pdl_enter();
   int j, i0;
   bool m[4];
   if (!swe_map(p, j, i0, m)) return;
@@ -63,7 +60,6 @@ __global__ void __launch_bounds__(SWE_THREADS)
 swe_k34_friction_u(B2SweParams p, const float* __restrict__ u, float* __restrict__ u_new,
                    const float* __restrict__ v, float* __restrict__ fe2, float* __restrict__ fn2,
                    int has_south) {
-  b2_pdl_enter();
   int j, i0;
   bool m[4];
   if (!swe_map(p, j, i0, m)) return;
@@ -73,7 +69,6 @@ swe_k34_friction_u(B2SweParams p, const float* __restrict__ u, float* __restrict
 __global__ void __launch_bounds__(SWE_THREADS)
 swe_k5_friction_v(B2SweParams p, float* __restrict__ v, const float* __restrict__ fe2,
                   const float* __restrict__ fn2) {
-  b2_pdl_enter();
   int j, i0;
   bool m[4];
   if (!swe_map(p, j, i0, m)) return;
@@ -107,7 +102,7 @@ static int swe_check(const B2SweParams* p) {
 static int b2_swe_fluxes(B2Comm* c, const B2SweParams* p, const float* h, const float* u, const float* v,
                   float* fe, float* fn, float* q, float* ke, cudaStream_t s) {
   if (int rc = swe_check(p)) return rc;
-  b2_launch(swe_k1_fluxes, swe_blocks(p), SWE_THREADS, 0, s, *p, h, u, v, fe, fn, q, ke);
+  swe_k1_fluxes<<<swe_blocks(p), SWE_THREADS, 0, s>>>(*p, h, u, v, fe, fn, q, ke);
   return swe_done(c, "swe_fluxes");
 }
 
@@ -115,7 +110,7 @@ static int b2_swe_tendencies(B2Comm* c, const B2SweParams* p, const float* h, fl
                       float* v, float* dh, float* du, float* dv, const float* fe, const float* fn,
                       const float* q, const float* ke, cudaStream_t s) {
   if (int rc = swe_check(p)) return rc;
-  b2_launch(swe_k2_tendencies, swe_blocks(p), SWE_THREADS, 0, s, *p, h, h_new, u, v, dh, du, dv, fe, fn, q, ke);
+  swe_k2_tendencies<<<swe_blocks(p), SWE_THREADS, 0, s>>>(*p, h, h_new, u, v, dh, du, dv, fe, fn, q, ke);
   return swe_done(c, "swe_tendencies");
 }
 
@@ -128,14 +123,14 @@ static int b2_swe_friction_u_fused(B2Comm* c, const B2SweParams* p, const float*
     b2_set_error("swe_friction_u_fused: u_new must not alias u (the update reads u's neighbours)");
     return B2_ERR_BAD_ARG;
   }
-  b2_launch(swe_k34_friction_u, swe_blocks(p), SWE_THREADS, 0, s, *p, u, u_new, v, fe2, fn2, has_south);
+  swe_k34_friction_u<<<swe_blocks(p), SWE_THREADS, 0, s>>>(*p, u, u_new, v, fe2, fn2, has_south);
   return swe_done(c, "swe_friction_u_fused");
 }
 
 static int b2_swe_friction_v(B2Comm* c, const B2SweParams* p, float* v, const float* fe2, const float* fn2,
                       cudaStream_t s) {
   if (int rc = swe_check(p)) return rc;
-  b2_launch(swe_k5_friction_v, swe_blocks(p), SWE_THREADS, 0, s, *p, v, fe2, fn2);
+  swe_k5_friction_v<<<swe_blocks(p), SWE_THREADS, 0, s>>>(*p, v, fe2, fn2);
   return swe_done(c, "swe_friction_v");
 }
 

@@ -186,8 +186,6 @@ _SIGNATURES = {
          POINTER(B2StatusRecord), c_void_p],
     ),
     "b2_abi_info": (c_int, [POINTER(c_int), c_int]),
-    "b2_pdl_enabled": (c_int, []),
-    "b2_set_pdl": (None, [c_int]),
     "b2_gemm_allreduce": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_void_p]),
     "b2_halo_exchange": (c_int, [c_void_p, POINTER(B2HaloDesc), c_void_p]),
     "b2_swe_multistep_ca": (

@@ -98,7 +98,7 @@ class ShallowWaterModel:
         #   "standalone"  4 stencil kernels + 3 fused exchanges, 32 passes (b2_swe.cu): the oracle the
         #                 default schedule is compared with, bit for bit.
         if pipeline is None:
-            pipeline = os.environ.get("MPI4JAX_B200_SWE_PIPELINE", "").strip().lower() or "ca"
+            pipeline = "ca"
         if pipeline not in ("ca", "standalone"):
             raise ValueError(f"unknown shallow-water pipeline {pipeline!r} (expected 'ca' or 'standalone')")
         self.pipeline = pipeline

@@ -9,7 +9,7 @@ REPO = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 LIB = os.path.join(REPO, "mpi4jax_b200", "_native", "libb2mpi.so")
 OUT = os.path.join(REPO, "profiles", "sass")
 WANT = {       # substring of the mangled name (with its length prefix where names share a stem) -> file
-    "9b2_k_halo9": "halo", "12b2_k_halo_ll": "halo_ll", "12b2_k_halo_ca": "halo_ca_deep_exchange",
+    "12b2_k_halo_ll": "halo_ll", "12b2_k_halo_ca": "halo_ca_deep_exchange",
     "swe_k1_fluxes": "swe_k1_fluxes", "swe_k2_tendencies": "swe_k2_tendencies", "swe_k34": "swe_k34_friction_u",
     "swe_k5": "swe_k5_friction_v", "swe_ca_bulk_k12": "swe_ca_bulk_k12", "swe_ca_bulk_fric": "swe_ca_bulk_fric",
     "swe_ca_tend_frame": "swe_ca_tend_frame", "swe_ca_fric_frame": "swe_ca_fric_frame",

@@ -98,31 +98,24 @@ def _share_path(path):
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("pdl", [0, 1], ids=["plain", "pdl"])
-def test_native_step_is_bitwise_reproducible(pdl):
+def test_native_step_is_bitwise_reproducible():
     """Two runs of the native step give identical bits (regression: the merged friction kernel
-    once updated u in place while neighbouring threads still read it), also with programmatic
-    dependent launch of the kernel chain."""
+    once updated u in place while neighbouring threads still read it)."""
     if not torch.cuda.is_available():
         pytest.skip("needs CUDA")
-    from mpi4jax_b200._src import native
 
     size = comm.Get_size()
     cfg = ShallowWaterConfig.for_resolution(1024 * max(1, size // 2), 2048)
-    native.lib.b2_set_pdl(pdl)
-    try:
-        runs = []
-        for _ in range(3):
-            model = ShallowWaterModel(cfg, comm=comm, device=comm.device, backend="native")
-            model.multistep(11)          # odd: exercises the ping-pong copy-back of h and u
-            m.flush()
-            runs.append([t.clone() for t in model.state])
-        for other in runs[1:]:
-            for name, a, b in zip("h u v dh du dv".split(), runs[0], other):
-                assert torch.equal(a, b), f"{name} differs between two identical runs"
-        assert all(torch.isfinite(t).all() for t in runs[0])
-    finally:
-        native.lib.b2_set_pdl(0)
+    runs = []
+    for _ in range(3):
+        model = ShallowWaterModel(cfg, comm=comm, device=comm.device, backend="native")
+        model.multistep(11)          # odd: exercises the ping-pong copy-back of h and u
+        m.flush()
+        runs.append([t.clone() for t in model.state])
+    for other in runs[1:]:
+        for name, a, b in zip("h u v dh du dv".split(), runs[0], other):
+            assert torch.equal(a, b), f"{name} differs between two identical runs"
+    assert all(torch.isfinite(t).all() for t in runs[0])
 
 
 @pytest.mark.gpu
