@@ -2,6 +2,9 @@
 
 * allreduce 1 KB - 1 GB, fp32 + bf16, every transport (ll / oneshot / twoshot / nvls / auto)
   next to NCCL on the same box                                   (configs 2)
+* reduce_scatter 1 KB - 1 GB input per rank, fp32 SUM, every transport (ll / oneshot / nvls / auto)
+  next to NCCL reduce_scatter_tensor; the allreduce fp32 rows at the same size are the cost of the
+  allreduce + slice workaround
 * allgather and alltoall 1 KB - 1 GB per-rank payload vs NCCL     (config 4)
 * bcast, reduce, gather, scatter (root = last rank) vs NCCL, scan (no NCCL counterpart)
 * sendrecv ring, halo exchange latency
@@ -9,7 +12,7 @@
 Timing: ``reps`` back-to-back ops captured in ONE CUDA graph, one replay timed with CUDA
 events on the launching stream (barrier + synchronize before), max over ranks -- i.e. the
 kernels' time, not the Python launch path.  Bus bandwidth uses the NCCL-tests conventions:
-allreduce S/t*2(P-1)/P, allgather/alltoall (P-1)/P * total/t.
+allreduce S/t*2(P-1)/P, allgather/alltoall/reduce_scatter (P-1)/P * total/t.
 
     python -m mpi4jax_b200.run -n 8 bench/collectives_sweep.py [--max-bytes 1073741824] [--out f.json]
 """
@@ -35,6 +38,8 @@ ap.add_argument("--out", default="gpurun_out/collectives_sweep.json")
 ap.add_argument("--quick", action="store_true", help="every fourth size")
 ap.add_argument("--skip-allreduce-algos", action="store_true", help="time only the automatic choice")
 ap.add_argument("--only-allreduce", action="store_true", help="stop after the allreduce tables")
+ap.add_argument("--only-reduce-scatter", action="store_true",
+                help="only the fp32 allreduce table and the reduce_scatter table")
 ap.add_argument("--only-p2p", action="store_true", help="only the p2p ring, barrier and halo lines")
 ap.add_argument("--max-blocks", type=int, default=0, help="override the collective grid cap")
 ap.add_argument("--nvls-pipeline", type=int, default=-1, help="0 / 1: software pipelining of the NVLS allreduce")
@@ -122,12 +127,22 @@ def time_nccl(fn, reps):
 
 sizes = [] if ns.only_p2p else [1 << k for k in range(10, 31, 2 if ns.quick else 1) if ns.min_bytes <= (1 << k) <= ns.max_bytes]
 result = {"world": size, "nvls": has_nvls, "allreduce": {}, "allgather": {}, "alltoall": {}, "p2p": {}}
+# what the numbers were measured on: the card and its power limit, read in the same run
+result["gpu"] = torch.cuda.get_device_name(dev) if dev.type == "cuda" else "cpu"
+try:
+    import subprocess
+
+    q = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit,clocks.max.sm", "--format=csv,noheader"],
+                       capture_output=True, text=True, timeout=30)
+    result["nvidia_smi_name_power_limit_max_sm_clock"] = q.stdout.strip().splitlines() or q.stderr.strip()[:120]
+except Exception as exc:  # pragma: no cover
+    result["nvidia_smi_name_power_limit_max_sm_clock"] = f"unavailable: {exc}"[:120]
 
 # ---------------------------------------------------------------- allreduce
 sym_pool = None
 if sizes and size > 1 and dev.type == "cuda":
     sym_pool = m.symmetric_empty((max(sizes),), torch.uint8, comm=comm)
-for dtype, dname in ((torch.float32, "fp32"), (torch.bfloat16, "bf16")):
+for dtype, dname in ((torch.float32, "fp32"),) + (() if ns.only_reduce_scatter else ((torch.bfloat16, "bf16"),)):
     table = {}
     for nbytes in sizes:
         x = torch.ones(nbytes // torch.empty((), dtype=dtype).element_size(), dtype=dtype, device=dev)
@@ -163,7 +178,38 @@ for dtype, dname in ((torch.float32, "fp32"), (torch.bfloat16, "bf16")):
         del x
     result["allreduce"][dname] = table
 
-if ns.only_allreduce:
+# ---------------------------------------------------------------- reduce_scatter (input per rank = nbytes)
+result["reduce_scatter"] = {}
+for nbytes in ([] if ns.only_allreduce else sizes):
+    if nbytes < 4 * size:
+        continue
+    blk = nbytes // 4 // size
+    x = torch.ones(size, blk, device=dev)
+    tot = x.numel() * 4
+    reps = reps_for(nbytes)
+    row = {}
+    for algo in ("auto", "ll", "oneshot", "nvls"):
+        if algo == "ll" and 2 * blk * 4 > (128 << 10):
+            continue
+        if algo == "nvls" and not has_nvls:
+            continue
+        try:
+            us = time_graph(lambda: m.reduce_scatter(x, MPI.SUM, comm=comm, algorithm=algo), reps)
+            row[algo] = {"us": round(us, 2), "busbw": round(tot * (size - 1) / size / us / 1e3, 1)}
+        except Exception as exc:
+            row[algo] = {"error": str(exc)[:120]}
+    if nccl is not None:
+        out = torch.empty(blk, device=dev)
+        flat = x.reshape(-1)
+        us = time_nccl(lambda: dist.reduce_scatter_tensor(out, flat, group=nccl), reps)
+        row["nccl"] = {"us": round(us, 2), "busbw": round(tot * (size - 1) / size / us / 1e3, 1)}
+        del out, flat
+    result["reduce_scatter"][str(nbytes)] = row
+    if rank == 0:
+        print("reduce_scatter", nbytes, {k: (v.get("us"), v.get("busbw")) for k, v in row.items()}, flush=True)
+    del x
+
+if ns.only_allreduce or ns.only_reduce_scatter:
     if rank == 0:
         os.makedirs(os.path.dirname(ns.out) or ".", exist_ok=True)
         with open(ns.out, "w") as f:

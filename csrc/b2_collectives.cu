@@ -13,8 +13,9 @@
 // Reduction collectives live in b2_reduce.cuh; this file adds the kernels that go through the
 // NVSwitch multicast object -- the NVLS allreduce of staged data (b2_k_allreduce_nvls), the
 // in-place allreduce of symmetric tensors (b2_k_allreduce_sym), the multicast bcast
-// (b2_k_bcast_mc), the reduce-to-root (b2_k_reduce_root_nvls) --, the size-based algorithm
-// selection and the grid cap that keeps every launch co-resident (coresident_blocks).
+// (b2_k_bcast_mc), the reduce-to-root (b2_k_reduce_root_nvls), the in-switch reduce-scatter
+// (b2_k_reduce_scatter_nvls) --, the size-based algorithm selection and the grid cap that keeps every
+// launch co-resident (coresident_blocks).
 #include <cstdio>
 #include <cstring>
 
@@ -23,6 +24,8 @@
 
 b2_reduce_launch_fn b2_reduce_table[B2_DTYPE_COUNT][B2_OP_COUNT];
 b2_ll_launch_fn b2_ll_table[B2_DTYPE_COUNT][B2_OP_COUNT];
+b2_rs_launch_fn b2_rs_table[B2_DTYPE_COUNT][B2_OP_COUNT];
+b2_rs_launch_fn b2_rs_ll_table[B2_DTYPE_COUNT][B2_OP_COUNT];
 void b2_register_reduce_group_0();
 void b2_register_reduce_group_1();
 void b2_register_reduce_group_2();
@@ -555,6 +558,85 @@ b2_k_reduce_root_nvls(const B2DevComm c, const B2ReduceArgs a) {
   b2_finish_bump(c.ticket, c.ticket + 1, 1u, gridDim.x);
 }
 
+
+// reduce-scatter (SUM, f32 / bf16 / f16): every rank stages the P pieces of a chunk, then reads the
+// in-switch sum of piece `rank` with multimem.ld_reduce straight into its output.  Next to the NVLS
+// allreduce there is no multimem.st broadcast, no second barrier and no copy out.
+template <int DT>
+__global__ void __launch_bounds__(B2_THREADS, 2)     // <= 64 registers: two CTAs per SM (coresident_blocks)
+b2_k_reduce_scatter_nvls(const B2DevComm c, const B2RSArgs a) {
+  const unsigned ticket = b2_ticket_read(c.ticket);
+  const size_t par = (size_t)(ticket & 1u) * c.stage_half;
+  unsigned e = b2_ld_volatile(c.epoch + blockIdx.x);
+  const char* in = (const char*)a.in;
+  char* out = (char*)a.out;
+  char* mine = c.stage[c.rank] + par;
+  const char* red = c.stage_mc + par + (size_t)c.rank * a.blk_stride;     // piece `rank`, through the switch
+  const size_t nb = a.blk_bytes, st = a.blk_stride;
+  const size_t nchunks = (nb + a.chunk - 1) / a.chunk;
+  const int t = threadIdx.x, nt = blockDim.x, P = c.size;
+#define CH_OFF(ch) ((ch) * a.chunk)
+#define CH_LEN(ch) ((nb - CH_OFF(ch) < a.chunk) ? (nb - CH_OFF(ch)) : a.chunk)
+  // software pipeline: the P pieces of the next chunk are staged while this one is reduced, in the
+  // SAME loop as the multimem.ld_reduce, so the switch round trips and the HBM loads overlap
+  size_t ch = blockIdx.x;
+  unsigned e_cur = e;
+  if (ch < nchunks) {
+#pragma unroll 1
+    for (int q = 0; q < P; ++q)
+      b2_copy_bytes<false>(mine + (size_t)q * st + CH_OFF(ch), in + (size_t)q * nb + CH_OFF(ch), CH_LEN(ch));
+    b2_barrier_arrive(c, ++e);
+    e_cur = e;
+  }
+  for (; ch < nchunks; ch += gridDim.x) {
+    const size_t nxt = ch + gridDim.x;
+    const bool more = nxt < nchunks;
+    const size_t off = CH_OFF(ch), len = CH_LEN(ch);
+    const size_t noff = more ? CH_OFF(nxt) : 0, nlen = more ? CH_LEN(nxt) : 0;
+    b2_barrier_wait(c, e_cur, a.opcode);              // every rank staged this chunk
+    const size_t nv = (len + 15) >> 4;
+    const size_t nvi = a.own_in ? (nlen >> 4) : 0;    // whole vectors of every next piece (own_in: no tails)
+    const size_t nmax = nv > nvi ? nv : nvi;
+    for (size_t base = 0; base < nmax; base += 2 * (size_t)nt) {
+      const size_t i0 = base + t, i1 = i0 + nt;
+      uint4 r0 = make_uint4(0, 0, 0, 0), r1 = r0;
+      if (i0 < nv) r0 = b2_mc_ld_reduce<DT>(red + off + (i0 << 4));
+      if (i1 < nv) r1 = b2_mc_ld_reduce<DT>(red + off + (i1 << 4));
+#pragma unroll 1
+      for (int q = 0; q < P; ++q) {
+        const char* src = in + (size_t)q * nb + noff;
+        char* dst = mine + (size_t)q * st + noff;
+        uint4 s0 = make_uint4(0, 0, 0, 0), s1 = s0;
+        if (i0 < nvi) s0 = b2_ld_stream16(src + (i0 << 4));
+        if (i1 < nvi) s1 = b2_ld_stream16(src + (i1 << 4));
+        if (i0 < nvi) b2_st16(dst + (i0 << 4), s0);
+        if (i1 < nvi) b2_st16(dst + (i1 << 4), s1);
+      }
+      if (i0 < nv) {
+        if ((i0 << 4) + 16 <= len) b2_st16(out + off + (i0 << 4), r0);
+        else b2_store_partial(out + off + (i0 << 4), r0, (int)(len - (i0 << 4)));
+      }
+      if (i1 < nv) {
+        if ((i1 << 4) + 16 <= len) b2_st16(out + off + (i1 << 4), r1);
+        else b2_store_partial(out + off + (i1 << 4), r1, (int)(len - (i1 << 4)));
+      }
+    }
+    if (more) {
+      if (!a.own_in)                                  // unaligned blocks: stage the next chunk byte-wise
+#pragma unroll 1
+        for (int q = 0; q < P; ++q)
+          b2_copy_bytes<false>(mine + (size_t)q * st + noff, in + (size_t)q * nb + noff, nlen);
+      b2_barrier_arrive(c, ++e);
+      e_cur = e;
+    }
+  }
+#undef CH_OFF
+#undef CH_LEN
+  __syncthreads();
+  if (t == 0) b2_st_volatile(c.epoch + blockIdx.x, e);
+  b2_finish_bump(c.ticket, c.ticket + 1, 1u, gridDim.x);
+}
+
 // ---------------------------------------------------------------------------
 // host helpers
 // ---------------------------------------------------------------------------
@@ -614,6 +696,7 @@ extern "C" size_t b2_stage_need(int opcode, int nranks, size_t blk_bytes) {
   switch (opcode) {
     case B2_OPC_ALLTOALL:
     case B2_OPC_SCATTER:
+    case B2_OPC_REDUCE_SCATTER:
       return stride * (size_t)nranks + 4096;
     default:
       return stride + 4096;
@@ -798,6 +881,83 @@ extern "C" int b2_scan(B2Comm* c, const void* in, void* out, size_t count, int d
   const size_t nbytes = count * b2_dtype_size(dtype);
   const int algo = (c->dev.size > 2 && nbytes > c->oneshot_max) ? B2_ALGO_TWOSHOT : B2_ALGO_ONESHOT;
   int rc = reduce_common(c, in, out, count, dtype, op, algo, 0, c->dev.rank + 1, 1, B2_OPC_SCAN, "scan", stream);
+  b2_debug_end(dbg, rc);
+  return rc;
+}
+
+// Reduce-scatter transports.  "auto" gives the same answer on every rank: it depends only on P, the
+// dtype, the op, multicast and the communicator's thresholds.  N = P x block is the input bytes per
+// rank, the quantity an allreduce of the same input compares against the same thresholds.
+static int reduce_scatter_common(B2Comm* c, const void* in, void* out, size_t count, int dtype, int op,
+                                 int algo, cudaStream_t stream) {
+  const char* name = "reduce_scatter";
+  b2_ensure_tables();
+  if (dtype < 0 || dtype >= B2_DTYPE_COUNT || op < 0 || op >= B2_OP_COUNT ||
+      b2_rs_table[dtype][op] == nullptr) {
+    b2_set_error("%s: unsupported dtype/op combination (dtype=%d, op=%d)", name, dtype, op);
+    return B2_ERR_BAD_ARG;
+  }
+  const size_t blk = count * b2_dtype_size(dtype);
+  if (blk == 0) return 0;
+  const int P = c->dev.size;
+  const size_t N = blk * (size_t)P;
+  const bool nvls_ok = c->dev.stage_mc != nullptr && op == B2_SUM &&
+                       (dtype == B2_F32 || dtype == B2_BF16 || dtype == B2_F16);
+  if (algo == B2_ALGO_AUTO) {
+    if (P > 1 && N <= c->ll_max && 2 * blk <= c->dev.lay.ll_cap) algo = B2_ALGO_LL;
+    else if (P > 2 && nvls_ok && N >= c->nvls_min) algo = B2_ALGO_NVLS;
+    else algo = B2_ALGO_ONESHOT;
+  }
+  if ((((uintptr_t)out) & 15) != 0) {
+    b2_set_error("%s: the output must be 16-byte aligned", name);
+    return B2_ERR_BAD_ARG;
+  }
+  B2RSArgs a;
+  a.in = in; a.out = out; a.blk_bytes = blk; a.blk_stride = round_up(blk, 16); a.chunk = 0;
+  a.own_in = ((((uintptr_t)in) & 15) == 0 && (blk & 15) == 0) ? 1 : 0;
+  a.opcode = B2_OPC_REDUCE_SCATTER;
+  int grid;
+  if (algo == B2_ALGO_LL) {
+    if (2 * blk > c->dev.lay.ll_cap) {
+      b2_set_error("%s: LL algorithm needs blocks of <= %zu bytes", name, c->dev.lay.ll_cap / 2);
+      return B2_ERR_BAD_ARG;
+    }
+    const size_t nv = (blk + 15) / 16;
+    grid = (int)((nv + B2_THREADS - 1) / B2_THREADS);
+    if (grid > c->sm_count) grid = c->sm_count;
+    if (grid < 1) grid = 1;
+    return finish_launch(c, b2_rs_ll_table[dtype][op](c->dev, a, grid, stream), name);
+  }
+  if (algo != B2_ALGO_ONESHOT && algo != B2_ALGO_NVLS) {
+    b2_set_error("%s: unknown algorithm %d (ll, oneshot or nvls)", name, algo);
+    return B2_ERR_BAD_ARG;
+  }
+  int rc = check_stage(c, B2_OPC_REDUCE_SCATTER, blk, name);
+  if (rc) return rc;
+  if (algo == B2_ALGO_NVLS) {
+    if (!nvls_ok) {
+      b2_set_error("%s: NVLS path needs a multicast-bound staging segment and SUM on f32/bf16/f16", name);
+      return B2_ERR_BAD_ARG;
+    }
+    const void* kern = dtype == B2_F32 ? (const void*)b2_k_reduce_scatter_nvls<B2_F32>
+                       : dtype == B2_BF16 ? (const void*)b2_k_reduce_scatter_nvls<B2_BF16>
+                                          : (const void*)b2_k_reduce_scatter_nvls<B2_F16>;
+    pick_chunks(c, blk, coresident_blocks(c, kern), &a.chunk, &grid);
+    if (dtype == B2_F32) b2_k_reduce_scatter_nvls<B2_F32><<<grid, B2_THREADS, 0, stream>>>(c->dev, a);
+    else if (dtype == B2_BF16) b2_k_reduce_scatter_nvls<B2_BF16><<<grid, B2_THREADS, 0, stream>>>(c->dev, a);
+    else b2_k_reduce_scatter_nvls<B2_F16><<<grid, B2_THREADS, 0, stream>>>(c->dev, a);
+    return finish_launch(c, cudaGetLastError(), name);
+  }
+  pick_chunks(c, blk, coresident_blocks(c, nullptr), &a.chunk, &grid);     // (typed kernel: one CTA per SM)
+  return finish_launch(c, b2_rs_table[dtype][op](c->dev, a, grid, stream), name);
+}
+
+extern "C" int b2_reduce_scatter(B2Comm* c, const void* in, void* out, size_t count, int dtype, int op,
+                                 int algo, cudaStream_t stream) {
+  char det[96];
+  snprintf(det, sizeof det, "with %zu items per rank", count);
+  B2DebugScope* dbg = b2_debug_begin(c, "Reduce_scatter_block", det, stream);
+  int rc = reduce_scatter_common(c, in, out, count, dtype, op, algo, stream);
   b2_debug_end(dbg, rc);
   return rc;
 }

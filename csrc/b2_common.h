@@ -16,7 +16,7 @@
 #include <cstddef>
 #include <cstdint>
 
-#define B2_ABI_VERSION 10   // bump whenever a struct shared with Python or a C signature changes
+#define B2_ABI_VERSION 11   // bump whenever a struct shared with Python or a C signature changes
 #define B2_MAX_RANKS 16          // ranks per NVLink domain we support (8 on HGX B200)
 #define B2_MAX_BLOCKS 1024       // max CTAs per collective launch (flag rows)
 #define B2_P2P_NSLOT 8           // ring slots per directed pair
@@ -83,7 +83,7 @@ struct B2StatusRecord {
 enum B2OpCode : int {
   B2_OPC_BARRIER = 0, B2_OPC_ALLREDUCE, B2_OPC_REDUCE, B2_OPC_SCAN, B2_OPC_ALLGATHER,
   B2_OPC_ALLTOALL, B2_OPC_BCAST, B2_OPC_GATHER, B2_OPC_SCATTER, B2_OPC_SEND, B2_OPC_RECV,
-  B2_OPC_SENDRECV, B2_OPC_HALO, B2_OPC_COUNT
+  B2_OPC_SENDRECV, B2_OPC_HALO, B2_OPC_REDUCE_SCATTER, B2_OPC_COUNT
 };
 
 static inline size_t b2_dtype_size(int dt) {

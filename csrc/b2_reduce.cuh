@@ -20,6 +20,7 @@
 #pragma once
 
 #include "b2_device.cuh"
+#include "b2_reduce_scatter.cuh"
 
 struct B2ReduceArgs {
   const void* in;
@@ -224,7 +225,9 @@ extern b2_ll_launch_fn b2_ll_table[B2_DTYPE_COUNT][B2_OP_COUNT];
 
 #define B2_REG(DT, T, OP)                               \
   b2_reduce_table[DT][OP] = &b2_launch_reduce<T, OP>;   \
-  b2_ll_table[DT][OP] = &b2_launch_ll<T, OP>;
+  b2_ll_table[DT][OP] = &b2_launch_ll<T, OP>;           \
+  b2_rs_table[DT][OP] = &b2_launch_rs<T, OP>;           \
+  b2_rs_ll_table[DT][OP] = &b2_launch_rs_ll<T, OP>;
 
 #define B2_REG_ARITH(DT, T) \
   B2_REG(DT, T, B2_SUM) B2_REG(DT, T, B2_PROD) B2_REG(DT, T, B2_MIN) B2_REG(DT, T, B2_MAX)

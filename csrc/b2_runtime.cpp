@@ -485,7 +485,8 @@ extern "C" long long b2_comm_get_option(B2Comm* c, const char* key) {
 
 static const char* opcode_name(int opc) {
   static const char* names[] = {"Barrier", "Allreduce", "Reduce", "Scan", "Allgather", "Alltoall",
-                                "Bcast", "Gather", "Scatter", "Send", "Recv", "Sendrecv", "Halo"};
+                                "Bcast", "Gather", "Scatter", "Send", "Recv", "Sendrecv", "Halo",
+                                "Reduce_scatter_block"};
   if (opc < 0 || opc >= B2_OPC_COUNT) return "Unknown";
   return names[opc];
 }

@@ -132,6 +132,10 @@ int b2_reduce(B2Comm* c, const void* in, void* out, size_t count, int dtype, int
               cudaStream_t stream);
 int b2_scan(B2Comm* c, const void* in, void* out, size_t count, int dtype, int op,
             cudaStream_t stream);
+// MPI_Reduce_scatter_block: `in` holds size blocks of `count` elements, rank r receives the reduction of
+// block r over all ranks in `out` (`count` elements)
+int b2_reduce_scatter(B2Comm* c, const void* in, void* out, size_t count, int dtype, int op, int algo,
+                      cudaStream_t stream);
 // `lay` (may be null = contiguous) describes a strided input; the pack is fused into the staging copy
 int b2_allgather(B2Comm* c, const void* in, void* out, size_t blk_bytes, const B2Strided* lay,
                  cudaStream_t stream);

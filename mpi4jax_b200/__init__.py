@@ -24,6 +24,7 @@ from ._src import (  # noqa: F401
     has_sycl_support,
     recv,
     reduce,
+    reduce_scatter,
     scan,
     scatter,
     send,
@@ -41,5 +42,5 @@ __all__ = [
     "allgather", "allreduce", "alltoall", "barrier", "bcast", "gather", "recv", "reduce",
     "scan", "scatter", "send", "sendrecv", "has_cuda_support", "has_sycl_support",
     "MPI", "jit", "compiled", "flush", "effects_barrier", "linear_transpose", "send_with_grad", "comm_reserve",
-    "symmetric_empty", "allreduce_",
+    "symmetric_empty", "allreduce_", "reduce_scatter",
 ]

@@ -25,6 +25,7 @@ from .collective_ops.bcast import bcast  # noqa: E402,F401
 from .collective_ops.gather import gather  # noqa: E402,F401
 from .collective_ops.recv import recv  # noqa: E402,F401
 from .collective_ops.reduce import reduce  # noqa: E402,F401
+from .collective_ops.reduce_scatter import reduce_scatter  # noqa: E402,F401
 from .collective_ops.scan import scan  # noqa: E402,F401
 from .collective_ops.scatter import scatter  # noqa: E402,F401
 from .collective_ops.send import send, send_with_grad  # noqa: E402,F401

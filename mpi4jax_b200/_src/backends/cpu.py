@@ -148,6 +148,11 @@ def alltoall(comm: Comm, x: torch.Tensor) -> torch.Tensor:
     return stack[:, comm.rank].clone()
 
 
+def reduce_scatter(comm: Comm, x: torch.Tensor, op_code: int) -> torch.Tensor:
+    # x: (P, *S).  The blocks travel as an alltoall, then the P received blocks are reduced in rank order.
+    return reduce_stack(alltoall(comm, x), op_code)
+
+
 def bcast(comm: Comm, x: torch.Tensor, root: int) -> torch.Tensor:
     buf = _bytes_view(x).clone()
     if comm.size > 1:

@@ -316,14 +316,14 @@ class NativeComm:
     def ensure_stage(self, opcode: int, blk_bytes: int) -> None:
         # same formula as b2_stage_need() (csrc/b2_collectives.cu), evaluated without leaving Python
         stride = (blk_bytes + 15) & ~15
-        mult = self.comm.size if opcode in (codes.OPC_ALLTOALL, codes.OPC_SCATTER) else 1
+        mult = self.comm.size if opcode in (codes.OPC_ALLTOALL, codes.OPC_SCATTER, codes.OPC_REDUCE_SCATTER) else 1
         need = stride * mult + 4096
         if need > self._stage_half:
             self._grow_stage(2 * need + 8192)
 
     def reserve(self, nbytes: int) -> None:
-        """Make sure collectives of up to ``nbytes`` per rank (alltoall / scatter: per peer block
-        times size) never have to grow the staging segment again.  Collective."""
+        """Make sure collectives of up to ``nbytes`` per rank (alltoall / scatter / reduce_scatter: per
+        peer block times size) never have to grow the staging segment again.  Collective."""
         stride = (int(nbytes) + 15) & ~15
         need = stride * self.comm.size + 4096
         if need > self._stage_half:
@@ -413,6 +413,17 @@ class NativeComm:
         rc = _lib().b2_allreduce(self.handle, x.data_ptr(), out.data_ptr(), x.numel(), dt, op_code,
                                  algo, self._stream())
         self._check(rc, "Allreduce")
+        return out
+
+    def reduce_scatter(self, x: torch.Tensor, op_code: int, algo: int = codes.ALGO_AUTO) -> torch.Tensor:
+        """MPI_Reduce_scatter_block: ``x`` is ``(size, *S)``; returns op over all ranks of block ``rank``."""
+        x, dt, op_code = _prep_reduce(x, op_code)
+        out = torch.empty(x.shape[1:], dtype=x.dtype, device=x.device)
+        blk = out.numel()
+        self.ensure_stage(codes.OPC_REDUCE_SCATTER, blk * x.element_size())
+        rc = _lib().b2_reduce_scatter(self.handle, x.data_ptr(), out.data_ptr(), blk, dt, op_code, algo,
+                                      self._stream())
+        self._check(rc, "Reduce_scatter_block")
         return out
 
     # -- symmetric tensors: user memory inside the symmetric heap ---------------------------------
@@ -642,7 +653,7 @@ def _nvtx_wrap(name: str, fn):
 #: ``MPI4JAX_B200_NVTX=1``: one NVTX range per op (visible in Nsight Systems timelines); the
 #: methods are left untouched otherwise, so the fast path pays nothing (SURVEY 5.1)
 NVTX_OPS = ("barrier", "allreduce", "reduce", "scan", "allgather", "alltoall", "bcast", "gather", "scatter",
-            "send", "recv", "sendrecv", "gemm_allreduce", "halo_exchange")
+            "reduce_scatter", "send", "recv", "sendrecv", "gemm_allreduce", "halo_exchange")
 if env_flag("MPI4JAX_B200_NVTX", False):
     for _name in NVTX_OPS:
         setattr(NativeComm, _name, _nvtx_wrap(_name, getattr(NativeComm, _name)))

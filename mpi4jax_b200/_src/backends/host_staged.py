@@ -86,6 +86,9 @@ class HostStagedComm:
     def allgather(self, x):
         return self._up(_cpu.allgather(self.comm, self._down(x)), x)
 
+    def reduce_scatter(self, x, op_code: int, algo: int = 0):
+        return self._up(_cpu.reduce_scatter(self.comm, self._down(x), op_code), x)
+
     def alltoall(self, x):
         return self._up(_cpu.alltoall(self.comm, self._down(x)), x)
 

@@ -136,6 +136,17 @@ def alltoall(comm: Comm, x: torch.Tensor) -> torch.Tensor:
     return out
 
 
+def reduce_scatter(comm: Comm, x: torch.Tensor, op_code: int, algo: int = codes.ALGO_AUTO) -> torch.Tensor:
+    _plain(x)
+    if x.is_cuda:
+        return comm._native_comm().reduce_scatter(x, op_code, algo)
+    done = _log(comm, "Reduce_scatter_block", f"with {x[0].numel() if x.dim() else 0} items per rank")
+    out = _cpu.reduce_scatter(comm, x, op_code)
+    if done:
+        done()
+    return out
+
+
 def bcast(comm: Comm, x: torch.Tensor, root: int) -> torch.Tensor:
     _plain(x)
     if x.is_cuda:

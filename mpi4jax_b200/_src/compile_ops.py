@@ -83,6 +83,30 @@ def _allreduce_backward(ctx, g):
 _allreduce.register_autograd(_allreduce_backward, setup_context=_allreduce_setup)
 
 
+@custom_op("mpi4jax_b200::reduce_scatter", mutates_args=())
+def _reduce_scatter(x: torch.Tensor, op: int, comm_id: int) -> torch.Tensor:
+    return _dispatch.reduce_scatter(_c(comm_id), x.contiguous(), op, codes.ALGO_AUTO)
+
+
+@_reduce_scatter.register_fake
+def _(x, op, comm_id):
+    return x.new_empty(x.shape[1:])
+
+
+def _reduce_scatter_setup(ctx, inputs, output):
+    _, ctx.op, ctx.comm_id = inputs
+
+
+def _reduce_scatter_backward(ctx, g):
+    if ctx.op != SUM.code:
+        raise NotImplementedError("The adjoint of reduce_scatter is only defined for SUM")
+    comm = _c(ctx.comm_id)
+    return torch.ops.mpi4jax_b200.allgather(g.contiguous(), ctx.comm_id, comm.Get_size()), None, None
+
+
+_reduce_scatter.register_autograd(_reduce_scatter_backward, setup_context=_reduce_scatter_setup)
+
+
 @custom_op("mpi4jax_b200::allgather", mutates_args=())
 def _allgather(x: torch.Tensor, comm_id: int, size: int) -> torch.Tensor:
     return _dispatch.allgather(_c(comm_id), x.contiguous())
@@ -267,7 +291,7 @@ def _sendrecv_backward(ctx, g):
 _sendrecv.register_autograd(_sendrecv_backward, setup_context=_sendrecv_setup)
 
 
-ALL_OPS = ("allreduce", "allgather", "alltoall", "bcast", "scan", "reduce", "gather_root", "gather_leaf",
+ALL_OPS = ("allreduce", "reduce_scatter", "allgather", "alltoall", "bcast", "scan", "reduce", "gather_root", "gather_leaf",
            "scatter", "barrier", "send", "recv", "sendrecv")
 ORDERED_EFFECT = False
 try:  # the ordered effect: AOTAutograd threads a token through these ops in program order
@@ -287,6 +311,11 @@ class compiled:
     @staticmethod
     def allreduce(x, op, *, comm=None):
         return torch.ops.mpi4jax_b200.allreduce(x, as_op(op).code, _register(comm))
+
+    @staticmethod
+    def reduce_scatter(x, op, *, comm=None):
+        """``x`` of shape ``(nproc, ...)`` -> this rank's reduced block (SUM is differentiable)."""
+        return torch.ops.mpi4jax_b200.reduce_scatter(x, as_op(op).code, _register(comm))
 
     @staticmethod
     def allgather(x, *, comm=None):

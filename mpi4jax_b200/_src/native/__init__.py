@@ -171,6 +171,8 @@ _SIGNATURES = {
     "b2_allreduce_sym": (c_int, [c_void_p, c_void_p, c_size_t, c_int, c_void_p]),
     "b2_reduce": (c_int, [c_void_p, c_void_p, c_void_p, c_size_t, c_int, c_int, c_int, c_void_p]),
     "b2_scan": (c_int, [c_void_p, c_void_p, c_void_p, c_size_t, c_int, c_int, c_void_p]),
+    # (comm, in, out, count = elements per block, dtype, op, algo, stream)
+    "b2_reduce_scatter": (c_int, [c_void_p, c_void_p, c_void_p, c_size_t, c_int, c_int, c_int, c_void_p]),
     "b2_allgather": (c_int, [c_void_p, c_void_p, c_void_p, c_size_t, POINTER(B2Strided), c_void_p]),
     "b2_alltoall": (c_int, [c_void_p, c_void_p, c_void_p, c_size_t, POINTER(B2Strided), c_void_p]),
     "b2_bcast": (c_int, [c_void_p, c_void_p, c_void_p, c_size_t, c_int, POINTER(B2Strided), c_void_p]),
@@ -206,7 +208,7 @@ _SIGNATURES = {
 
 
 #: must equal B2_ABI_VERSION in csrc/b2_common.h
-ABI_VERSION = 10
+ABI_VERSION = 11
 _ABI_FIELDS = ("abi_version", "sizeof_status_record", "sizeof_halo_desc", "sizeof_swe_params",
                "sizeof_swe_state", "sizeof_error_record", "max_ranks", "p2p_nslot", "sizeof_swe_ca")
 

@@ -41,5 +41,6 @@ ALGO_BY_NAME = {
 # enum B2OpCode (subset used from Python)
 OPC_ALLREDUCE, OPC_REDUCE, OPC_SCAN, OPC_ALLGATHER, OPC_ALLTOALL = 1, 2, 3, 4, 5
 OPC_BCAST, OPC_GATHER, OPC_SCATTER = 6, 7, 8
+OPC_REDUCE_SCATTER = 13
 
 ANY = -1  # ANY_SOURCE / ANY_TAG on the wire

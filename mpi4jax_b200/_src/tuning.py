@@ -1,12 +1,18 @@
 """Per-world-size transport thresholds of the GPU collectives.
 
 The native library picks a transport per call from a handful of byte thresholds
-(csrc/b2_collectives.cu: reduce_common, b2_bcast):
+(csrc/b2_collectives.cu: reduce_common, reduce_scatter_common, b2_bcast):
 
-* ``ll_max``        allreduce: flag-in-data (LL) kernel up to this many bytes
+* ``ll_max``        allreduce / reduce_scatter: flag-in-data (LL) kernel up to this many bytes
 * ``oneshot_max``   reductions without multicast: one-shot pull up to here, two-shot beyond
-* ``nvls_min``      allreduce / reduce: in-switch (NVLS) reduction from this size on (world size > 2)
+* ``nvls_min``      allreduce / reduce / reduce_scatter: in-switch (NVLS) reduction from this size on
+                    (world size > 2)
 * ``bcast_mc_min``  bcast: one ``multimem.st`` stream from the root from this size on (world size > 2)
+
+reduce_scatter compares its whole input per rank (P blocks) with ``ll_max`` and ``nvls_min``, the bytes an
+allreduce of the same input compares; below ``nvls_min``, or without multicast, it uses its one-shot pull.
+These thresholds were measured for allreduce only; ``bench/collectives_sweep.py`` records every forced
+reduce_scatter transport next to them, so a later change can give reduce_scatter keys of its own.
 
 Which transport wins where depends on the number of ranks (at 2 ranks a one-shot pull beats the
 switch at every size: each GPU has to serve P + 1 streams for an in-switch allreduce) and on the box.

@@ -159,7 +159,8 @@ def fold(parts, op) -> torch.Tensor:
 
 def comm_reserve(nbytes: int, *, comm: Optional[_comm.Comm] = None) -> None:
     """Pre-size the GPU staging buffers of ``comm`` (default communicator if None) for collectives
-    of up to ``nbytes`` per rank, so that no later call has to grow them.  Growth is collective and
+    of up to ``nbytes`` per rank (alltoall, scatter and reduce_scatter: per block), so that no later
+    call has to grow them.  Growth is collective and
     impossible during CUDA-graph capture; ``mpi4jax_b200.jit`` avoids it by running a function once
     eagerly, ``comm_reserve`` is the explicit alternative.  A no-op on CPU communicators."""
     if comm is None:

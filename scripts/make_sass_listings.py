@@ -20,6 +20,7 @@ WANT = {       # substring of the mangled name (with its length prefix where nam
     "b2_k_reduce_chunkedIfLi0": "reduce_chunked_f32_sum",
     "b2_k_reduce_chunkedI13__nv_bfloat16Li0": "reduce_chunked_bf16_sum",
     "b2_k_gemm": "gemm_allreduce_tcgen05",
+    "b2_k_reduce_scatter_nvlsILi0": "reduce_scatter_nvls_f32", "b2_k_reduce_scatter_llIfLi0": "reduce_scatter_ll_f32_sum",
 }
 HEADER = """# SASS listings (cuobjdump -sass libb2mpi.so, sm_100a)
 
